@@ -155,6 +155,28 @@ def measured_peak():
         return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
 
 
+DUMP_SAMPLE = 1 << 20      # --dump-outputs: elements kept of a larger output (at most 8 MB per array as float64)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write each output of the timed path's last step as <out_dir>/<name>.npy, so that two builds run with the
+    same arguments (hence the same inputs) can be compared output for output.  Bytes become float32, wider integers float64
+    (int32 buffers hold u32 words), both exact.  An output of more than DUMP_SAMPLE elements is cut down to the elements at a
+    fixed, seeded set of flat positions, the same in every run."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = torch.as_tensor(a)
+        if a.numel() > DUMP_SAMPLE:
+            pos = np.sort(np.random.default_rng(1).choice(a.numel(), DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[torch.from_numpy(pos).to(a.device)]
+        h = a.cpu().numpy()
+        if h.dtype == np.int32:
+            h = h.view(np.uint32)
+        np.save(os.path.join(out_dir, name + ".npy"), h.astype(np.float32 if h.dtype.itemsize == 1 else np.float64))
+
+
 def ncu_traffic(workload, batch, db_format):
     """dram bytes per launch of the multiply kernel from the committed ncu --set full capture of this configuration, if any
     (profiles/roofline_traffic.json; key = workload, queries per step, database format)."""
@@ -279,7 +301,7 @@ class CpuFullQuery:
 
     def one(self):
         t0 = time.perf_counter()
-        self.P.process_query(self.pp, self.q, self.db)
+        self.response = self.P.process_query(self.pp, self.q, self.db)
         return time.perf_counter() - t0
 
     def sample(self, n):
@@ -296,6 +318,8 @@ def run_reference_arm(args, kw, workload_name, rank, world):
         dt = cpu.one()                       # a step = one full process_query on the host cores
         if i >= args.warmup:
             per_step.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"responses": cpu.response.reshape(1, -1)})
     sec = sum(per_step) / len(per_step)
     qps = 1.0 / sec
     cores, sample = cpu.cores, cpu.sample(len(per_step))
@@ -349,6 +373,8 @@ def kernel_workload(args):
         b = torch.from_numpy(hb.view(np.int32)).cuda()
         out = torch.zeros(rows, dtype=torch.int32, device="cuda")
         ms = timed(lambda: check(LIB.b200pir_dpir_matvec_packed_dev(m._h, b.data_ptr(), out.data_ptr(), 0)))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"dpir_matvec": out})
         alg = 4 * rows * cols + 12 * cols + 4 * rows
         ho = np.zeros(rows, dtype=np.uint32)
         t1 = time.perf_counter()
@@ -379,11 +405,14 @@ def kernel_workload(args):
         count = 1 << 16
         res = {}
         for poly_len, fn in ((2048, LIB.b200pir_ntt32_dev), (4096, LIB.b200pir_ntt4096_dev)):
-            x = torch.randint(0, Q1, (count * 2 * poly_len,), dtype=torch.int32, device="cuda")
+            x = torch.randint(0, Q1, (count * 2 * poly_len,), dtype=torch.int32, device="cuda",
+                              generator=torch.Generator(device="cuda").manual_seed(poly_len))
             for name, inv in (("forward", 0), ("inverse", 1)):
                 if inv:
                     check(fn(G._h, x.data_ptr(), count, 0))               # inverse timed on canonical transform outputs
                 ms = timed(lambda: check(fn(G._h, x.data_ptr(), count, inv)))
+                if args.dump_outputs:                                     # the transforms run in place: x is the output
+                    dump_outputs(args.dump_outputs, {"ntt%d_%s" % (poly_len, name): x})
                 byt = 2 * count * 2 * poly_len * 4
                 res["%d_%s" % (poly_len, name)] = {"ms": ms, "polys_per_s": count / ms * 1e3, "GB/s_u32": byt / ms / 1e6,
                                                    "frac_of_hbm_peak_u32": byt / ms / 1e6 / peak}
@@ -448,6 +477,10 @@ def main():
                          "on an unsharded copy of the same database with the single-GPU path and compares the response bytes)")
     ap.add_argument("--steps-only", action="store_true",
                     help="profiling aid: skip the single-query latency probe and the e2e leg (clean ncu launch lists)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (for the Spiral workloads the response bytes of "
+                         "every query of the step) as DIR/<name>.npy in float32 / float64; an output of more than 2^20 elements is "
+                         "cut to a fixed, seeded sample")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
@@ -750,6 +783,15 @@ def main():
     clocks = sampler.stop(t_wall0, t_wall1)
     launches = LIB.b200pir_kernel_launches() - launches0
     ms_total = ev0.elapsed_time(ev1)
+    if args.dump_outputs:
+        # the responses of the last timed step, rank by rank; taken now, before the passes below reuse d_out
+        responses = d_out
+        if dist is not None:
+            responses = torch.empty(N * d_out.numel(), dtype=torch.uint8, device="cuda")
+            dist.all_gather_into_tensor(responses, d_out)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"responses": responses.reshape(B, rb)})
+        del responses
     if args.timeline and N > 1 and exchange == "ce":
         # where a step's time goes on this rank's streams (a separate, short pass; printed by every rank to stderr)
         tl_on[0] = True

@@ -1,33 +1,15 @@
-// The tcgen05 descriptors built by sdk_b200/csrc/tc5_layout.cuh, compared field by field with the bit-field structs of
-// the vendored CUTLASS headers (cute/arch/mma_sm100_desc.hpp).  Host-only; compiled with nvcc -I<cutlass>/include.
+// The tcgen05 descriptors built by sdk_b200/csrc/tc5_layout.cuh, printed in the format of tests/golden/tc5_descriptors.json
+// (the same fields packed by CUTLASS's bit-field structs, tests/golden/make_tc5_descriptors.cu).  Host-only; compiled with nvcc.
 #include <cstdio>
 #include <cstdint>
-#include <cute/arch/mma_sm100_desc.hpp>
 #include "../../sdk_b200/csrc/tc5_layout.cuh"
 int main() {
-  int bad = 0;
-  cute::UMMA::InstrDescriptor d = {};
-  d.desc_ = 0;
-  d.c_format_ = uint8_t(cute::UMMA::CFormat::S32);
-  d.a_format_ = uint8_t(cute::UMMA::S8Format::UINT8);
-  d.b_format_ = uint8_t(cute::UMMA::S8Format::UINT8);
-  d.a_major_ = uint8_t(cute::UMMA::Major::K);
-  d.b_major_ = uint8_t(cute::UMMA::Major::K);
-  d.n_dim_ = b200pir::TC5_N >> 3;
-  d.m_dim_ = b200pir::TC5_M >> 4;
-  if (d.desc_ != b200pir::tc5_instr_desc()) { printf("instr desc %08x vs %08x\n", d.desc_, b200pir::tc5_instr_desc()); bad++; }
+  printf("{\"instr_desc\": \"0x%08x\",\n \"smem_desc\": {", b200pir::tc5_instr_desc());
+  const char* sep = "";
   for (uint32_t addr : {0x0u, 0x400u, 0x12340u, 0x3FFF0u}) {
-    cute::UMMA::SmemDescriptor s;
-    s.desc_ = 0;
-    s.start_address_ = addr >> 4;
-    s.leading_byte_offset_ = b200pir::TC5_LBO >> 4;
-    s.stride_byte_offset_ = b200pir::TC5_SBO >> 4;
-    s.version_ = 1;
-    s.base_offset_ = 0;
-    s.lbo_mode_ = 0;
-    s.layout_type_ = uint8_t(cute::UMMA::LayoutType::SWIZZLE_NONE);
-    if (s.desc_ != b200pir::tc5_smem_desc(addr)) { printf("smem desc %016llx vs %016llx\n", (unsigned long long)s.desc_, (unsigned long long)b200pir::tc5_smem_desc(addr)); bad++; }
+    printf("%s\"0x%x\": \"0x%016llx\"", sep, addr, (unsigned long long)b200pir::tc5_smem_desc(addr));
+    sep = ", ";
   }
-  printf(bad ? "descriptor mismatch\n" : "descriptors ok\n");
-  return bad;
+  printf("}}\n");
+  return 0;
 }
