@@ -1,4 +1,6 @@
-// Pipe-rate microbenchmarks on sm_100a: legacy mma.sync variants and integer ops used by the NTT butterflies.
+// Pipe-rate microbenchmarks on sm_100a: legacy mma.sync variants, the integer ops used by the NTT butterflies and the FP64 ops
+// of a Shoup quotient taken on the FP64 pipe (bfly.cu kinds 4..7), alone and interleaved with mad.lo to show whether the two
+// pipes issue concurrently.
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o pipes pipes.cu ; prints per-SM per-clock rates.
 #include <cstdio>
 #include <cstdint>
@@ -104,6 +106,31 @@ __global__ void k_int(unsigned* out, unsigned seed, unsigned m) {
   out[blockIdx.x * blockDim.x + threadIdx.x] = s;
 }
 
+// FP64 ops: 8 independent chains per thread.  OP 3 interleaves one mad.lo.u32 chain step with one fma.rm.f64 chain step.
+template <int OP>
+__global__ void k_f64(unsigned* out, unsigned seed, double m) {
+  double x[8];
+  unsigned u[8];
+#pragma unroll
+  for (int j = 0; j < 8; j++) { x[j] = 1.0 + (seed + j * 77u + threadIdx.x) * 0x1p-40; u[j] = seed + j * 77u + threadIdx.x; }
+  for (int it = 0; it < ITER; it++) {
+#pragma unroll
+    for (int j = 0; j < 8; j++) {
+      if (OP == 0) asm volatile("fma.rn.f64 %0, %0, %1, %2;" : "+d"(x[j]) : "d"(m), "d"(-m));
+      if (OP == 1) asm volatile("fma.rm.f64 %0, %0, %1, %2;" : "+d"(x[j]) : "d"(m), "d"(-m));
+      if (OP == 2) asm volatile("add.f64 %0, %0, %1;" : "+d"(x[j]) : "d"(m));
+      if (OP == 3) {
+        asm volatile("mad.lo.u32 %0, %0, %1, %2;" : "+r"(u[j]) : "r"(seed), "r"(seed));
+        asm volatile("fma.rm.f64 %0, %0, %1, %2;" : "+d"(x[j]) : "d"(m), "d"(-m));
+      }
+    }
+  }
+  unsigned s = 0;
+#pragma unroll
+  for (int j = 0; j < 8; j++) s ^= (unsigned)__double2loint(x[j]) ^ u[j];
+  out[blockIdx.x * blockDim.x + threadIdx.x] = s;
+}
+
 template <typename F>
 float time_ms(F launch) {
   cudaEvent_t a, b;
@@ -143,6 +170,10 @@ int main() {
   rep("mul.wide.u32 (+xor)", time_ms([&] { k_int<4><<<ctas, thr>>>((unsigned*)buf, 3, 12345677u); }), 32, 8);
   rep("mulhi+add+min (3 instr)", time_ms([&] { k_int<5><<<ctas, thr>>>((unsigned*)buf, 3, 12345677u); }), 32, 24);
   rep("mad+add (2 instr)", time_ms([&] { k_int<6><<<ctas, thr>>>((unsigned*)buf, 3, 12345677u); }), 32, 16);
+  rep("fma.rn.f64", time_ms([&] { k_f64<0><<<ctas, thr>>>((unsigned*)buf, 3, 1.0000001); }), 32, 8);
+  rep("fma.rm.f64", time_ms([&] { k_f64<1><<<ctas, thr>>>((unsigned*)buf, 3, 1.0000001); }), 32, 8);
+  rep("add.f64", time_ms([&] { k_f64<2><<<ctas, thr>>>((unsigned*)buf, 3, 1.0000001); }), 32, 8);
+  rep("mad.lo.u32 + fma.rm.f64 (2)", time_ms([&] { k_f64<3><<<ctas, thr>>>((unsigned*)buf, 3, 1.0000001); }), 32, 16);
   CK(cudaDeviceSynchronize());
   CK(cudaGetLastError());
   return 0;

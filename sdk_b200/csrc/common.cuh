@@ -65,6 +65,14 @@ __device__ __forceinline__ uint32_t gadget_digit(uint64_t v, int k, int bits, ui
   const uint32_t w = __funnelshift_rc(__funnelshift_rc(lo, hi, sh), 0u, sh > 32 ? sh - 32 : 0);
   return w & (uint32_t)mask;
 }
+// Number of leading gadget digits that can be non-zero for values v <= bound: digit k of every such v is zero once
+// bound < 2^(k bits).  With modulus_log2 = 56 and t = 8 (bits = 8), digit 7 covers bits 56..63 and is always zero because
+// q0 q1 < 2^56.  Its forward transform is then zero mod q, so callers that reduce their accumulators mod q may skip it.
+__device__ __forceinline__ int gadget_live_digits(int t, int bits, uint64_t bound) {
+  int k = 0;
+  while (k < t && k * bits < 64 && (bound >> (k * bits)) != 0) k++;
+  return k;
+}
 
 __device__ __forceinline__ uint4 ld_stream_v4(const uint4* p) {
   uint4 r;

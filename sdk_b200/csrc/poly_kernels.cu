@@ -211,7 +211,9 @@ __device__ __forceinline__ void digits_mac_impl(uint64_t (&acc)[ROWS][8], int& c
   }
 }
 
-// one warp-uniform branch per call (not per digit): the byte-permute and the funnel-shift digit extraction as two loop bodies
+// one warp-uniform branch per call (not per digit): the byte-permute and the funnel-shift digit extraction as two loop bodies.
+// The expansion passes ndig = gadget_live_digits(t, bits, q0 q1): its values are <= q0 q1, so the digits it leaves out are
+// zero and would add only multiples of q to the accumulators, which are reduced mod q.
 template <int ROWS, bool SM>
 __device__ __forceinline__ void digits_mac(uint64_t (&acc)[ROWS][8], int& cnt, const uint64_t (&v)[8], int ndig,
                                            int bits, const uint32_t* c0, size_t col_step, size_t row_step,
@@ -422,7 +424,8 @@ __device__ __forceinline__ uint32_t digit_diff(uint64_t vh, uint64_t vi, int k, 
 // Same step as k_fold_res on the relaxed-range transforms (ntt_core.cuh "lz"): no per-butterfly range correction in the
 // forward transforms (outputs < 16q feed the 64-bit multiply-accumulate directly: 16 products of < 2^32 x < 2^28 fit),
 // no halving in the inverse transform, byte-permute digit extraction when bits_per = 8, 32-bit Barrett in the CRT lift.
-// Tried on top of this and measured without gain (S8, 16 queries; fold stage 3.53 ms): pass C / D twiddles held in registers at
+// Digits that are zero for every value < q0 q1 (digit 7 of the t = 8, 8-bit gadget) are skipped: fold stage 3.53 -> 3.26 ms
+// (S8, 16 queries, B200).  Tried before that and measured without gain (fold stage 3.53 ms): pass C / D twiddles held in registers at
 // 2 CTAs per SM (3.60 ms: 35 % less shared-memory traffic, so that is not the limit), key columns prefetched into L1 before the
 // pair's transforms (3.60 ms: the L2 latency ncu attributes to the multiply-accumulate is covered by the other CTAs).  The
 // kernel runs at ~80 % of its integer-multiply-pipe bound (DESIGN.md 4.3).
@@ -462,6 +465,9 @@ k_fold_res_lz(DevParams P, const uint32_t* __restrict__ in, uint32_t* __restrict
   const size_t row_step = (size_t)cols * 2 * POLY;
   const uint64_t mask = (1ull << bits) - 1;
   const uint32_t q = g.q;
+  // the CRT-lifted coefficients are < q0 q1: digits from ndig on are zero in both ciphertexts, so their differences (q) transform
+  // to multiples of q and add nothing mod q to the accumulators
+  const int ndig = gadget_live_digits(t_gsw, bits, P.modulus);
 
   uint64_t acc[2][8];
 #pragma unroll
@@ -481,7 +487,7 @@ k_fold_res_lz(DevParams P, const uint32_t* __restrict__ in, uint32_t* __restrict
     const uint32_t* c0 = C + ((size_t)rho * 2 + g.n) * POLY + g.tid * 8;       // key-matrix column of digit k: rho + 2k
     int k = 0;
 #pragma unroll 1
-    for (; k + 1 < t_gsw; k += 2) {
+    for (; k + 1 < ndig; k += 2) {
       uint32_t x0[8], x1[8];
 #pragma unroll
       for (int a = 0; a < 8; a++) {
@@ -502,7 +508,7 @@ k_fold_res_lz(DevParams P, const uint32_t* __restrict__ in, uint32_t* __restrict
         for (int e = 0; e < 8; e++) acc[r][e] += (uint64_t)x1[e] * cv[e];
       }
     }
-    if (k < t_gsw) {                            // odd t_gsw: last digit alone
+    if (k < ndig) {                             // odd digit count: last digit alone
       uint32_t x0[8];
 #pragma unroll
       for (int a = 0; a < 8; a++) x0[a] = digit_diff<BYTE>(vh[a], vi[a], k, bits, mask, q);
@@ -652,7 +658,7 @@ __global__ void __launch_bounds__(CTA, 1) k_expand_round(DevParams P, uint32_t* 
     for (int a = 0; a < 8; a++) vv[a] = autom[a * 256 + g.tid];
     // gadget_invert_rdim(.., rdim = 1): digit k -> key column k  (server.rs:82-89)
     const uint32_t* c0 = W + (size_t)g.n * POLY + g.tid * 8;
-    digits_mac<2, true>(acc, cnt, vv, t_exp, bits, c0, (size_t)2 * POLY, (size_t)t_exp * 2 * POLY, g);
+    digits_mac<2, true>(acc, cnt, vv, gadget_live_digits(t_exp, bits, P.modulus), bits, c0, (size_t)2 * POLY, (size_t)t_exp * 2 * POLY, g);
   }
 #pragma unroll
   for (int rho = 0; rho < 2; rho++) {
@@ -770,7 +776,7 @@ k_expand_round_pair(DevParams P, uint32_t* v, size_t v_stride, ExpandRound R, co
 #pragma unroll
       for (int a = 0; a < 8; a++) vv[a] = autom[a * 256 + g.tid];
       const uint32_t* c0 = W + (size_t)g.n * POLY + g.tid * 8;
-      digits_mac<2, true>(acc, cnt, vv, t_exp, bits, c0, (size_t)2 * POLY, (size_t)t_exp * 2 * POLY, g);
+      digits_mac<2, true>(acc, cnt, vv, gadget_live_digits(t_exp, bits, P.modulus), bits, c0, (size_t)2 * POLY, (size_t)t_exp * 2 * POLY, g);
     }
     uint32_t* dst = half ? vo : vi;
 #pragma unroll
@@ -897,7 +903,7 @@ k_expand_round_res(DevParams P, uint32_t* v, size_t v_stride, const uint32_t* __
 #pragma unroll
       for (int a = 0; a < 8; a++) vv[a] = autom[a * 256 + g.tid];
       const uint32_t* c0 = W + (size_t)g.n * POLY + g.tid * 8;
-      digits_mac<2, true>(acc, cnt, vv, t_exp, bits, c0, (size_t)2 * POLY, (size_t)t_exp * 2 * POLY, g);
+      digits_mac<2, true>(acc, cnt, vv, gadget_live_digits(t_exp, bits, P.modulus), bits, c0, (size_t)2 * POLY, (size_t)t_exp * 2 * POLY, g);
     }
     // row 1 automorphism = slot permutation (see k_expand_round); gather before any thread overwrites v[i]
     uint32_t yy[8];
