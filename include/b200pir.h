@@ -95,6 +95,18 @@ int b200pir_db_upsert_item(b200pir_ctx* ctx, b200pir_db* db, uint64_t slice, uin
  * of item db_idx (at most instances*n^2*bytes_per_chunk, zero padded); chunk c becomes the item polynomial of slice c
  * (convert_pt_to_poly :278-299: coefficient i = byte i, recenter_mod, NTT; pack_ntt_poly :34-41), all on the GPU. */
 int b200pir_db_update_item_raw(b200pir_ctx* ctx, b200pir_db* db, uint64_t db_idx, const uint8_t* data, size_t len);
+/* lib/server/src/db/loading.rs:361-377 update_many_items (the /update-row body): entries [u32 BE chunk_len][u32 BE db_idx]
+ * [chunk_len - 4 raw bytes], back to back; each entry is update_item (:301-315) -> update_item_raw (:317-359).
+ * largest_update (may be NULL) receives the longest entry's chunk_len, as the handler reports it.
+ * Entries are checked in body order with the codes and messages of b200pir_db_update_item_raw: a truncated length prefix, a
+ * chunk_len below 4 or past the end of the body, a chunk_len above 4 + instances*n^2*bytes_per_chunk and a db_idx >= num_items
+ * each give B200PIR_E_SHAPE, with every entry before the bad one written and none after it (the reference's serial loop).  The
+ * last entry of an item wins.  On a sharded database entries of other GPUs' rows are checked but not written.  The whole body
+ * is applied under the context lock and finished before the call returns, so concurrent queries see the database as it was
+ * before the call or as the call leaves it, never halfway.
+ * Entries are converted and placed in groups of at most 4096 items or 32 MiB of raw bytes (one fused kernel launch each),
+ * staged through two pinned buffers owned by the context: they grow on first use, later calls allocate nothing. */
+int b200pir_db_update_many_items(b200pir_ctx* ctx, b200pir_db* db, const uint8_t* body, size_t len, uint64_t* largest_update);
 /* Synthetic database generated on the GPU: plaintext coefficient = splitmix64(seed, ((slice*items+item)*2048+z)) % p,
  * then recenter_mod / NTT / pack as generate_random_db_and_get_item does (server.rs:223-275). */
 int b200pir_db_fill_synthetic(b200pir_ctx* ctx, b200pir_db* db, uint64_t seed);

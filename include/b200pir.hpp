@@ -88,6 +88,12 @@ struct Database {
   void upsert_item(uint64_t slice, uint64_t item_idx, const uint64_t* poly) {
     check(b200pir_db_upsert_item(params.ctx, h, slice, item_idx, poly));
   }
+  // lib/server/src/db/loading.rs:361-377 update_many_items: returns largest_update
+  uint64_t update_many_items(const uint8_t* body, size_t len) {
+    uint64_t largest = 0;
+    check(b200pir_db_update_many_items(params.ctx, h, body, len, &largest));
+    return largest;
+  }
 };
 
 namespace ntt {

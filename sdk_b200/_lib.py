@@ -43,6 +43,7 @@ def _load():
         "b200pir_db_load_raw_file": (C.c_int, [vp, vp, C.c_char_p]),
         "b200pir_db_upsert_item": (C.c_int, [vp, vp, C.c_uint64, C.c_uint64, u64p]),
         "b200pir_db_update_item_raw": (C.c_int, [vp, vp, C.c_uint64, u8p, C.c_size_t]),
+        "b200pir_db_update_many_items": (C.c_int, [vp, vp, u8p, C.c_size_t, C.POINTER(C.c_uint64)]),
         "b200pir_db_fill_synthetic": (C.c_int, [vp, vp, C.c_uint64]),
         "b200pir_db_info": (C.c_int, [vp, C.POINTER(C.c_int), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "b200pir_db_present_items": (C.c_int, [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),

@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libb200pir.so")
 SOURCES = ["api.cu", "poly_kernels.cu", "mul_kernels.cu", "imma_kernels.cu", "wire_kernels.cu", "tc5_kernels.cu", "dpir_gemm.cu"]
-HEADERS = ["common.cuh", "kernels.h", "ntt_core.cuh", "tc5_layout.cuh", "tc5_ptx.cuh", "ntt_core4096.cuh", "ntt_tables.hpp", os.path.join("..", "..", "include", "b200pir.h")]
+HEADERS = ["common.cuh", "kernels.h", "item_write.cuh", "ntt_core.cuh", "tc5_layout.cuh", "tc5_ptx.cuh", "ntt_core4096.cuh", "ntt_tables.hpp", os.path.join("..", "..", "include", "b200pir.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--extended-lambda",
               "-Xcompiler", "-fPIC", "-ccbin", "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"]
 

@@ -9,6 +9,7 @@
 #include <algorithm>
 #include <cmath>
 #include <memory>
+#include <cstdint>
 #include <cstring>
 #include <condition_variable>
 #include <chrono>
@@ -16,6 +17,7 @@
 #include <mutex>
 #include <set>
 #include <string>
+#include <unordered_set>
 #include <utility>
 #include <vector>
 
@@ -71,6 +73,36 @@ struct DevBuf {
   DevBuf& operator=(const DevBuf&) = delete;
 };
 
+// Bulk writes (update_many_items, update_item_raw, load_raw_file) go through the fused kernel of item_write.cuh in groups of at
+// most kWriteGroupItems items, closed once their raw bytes reach kWriteGroupBytes (b200pir.h).
+constexpr size_t kWriteGroupItems = 4096;
+constexpr size_t kWriteGroupBytes = (size_t)32 << 20;
+
+// One staging buffer of the write path: [ItemWrite x count][raw bytes], pinned on the host and mirrored on the device.  A
+// context owns two and alternates, so that the host fills one while the kernel of the previous group reads the other.
+struct WriteStage {
+  uint8_t* host = nullptr;
+  size_t cap = 0;
+  DevBuf<uint8_t> dev;
+  cudaEvent_t copied = nullptr;     // the last copy out of `host` has finished: it may be refilled
+  void ensure(size_t bytes) {
+    if (!copied) B200_CUDA(cudaEventCreateWithFlags(&copied, cudaEventDisableTiming));
+    B200_CUDA(cudaEventSynchronize(copied));
+    if (bytes <= cap) return;
+    bytes = std::max(bytes, (size_t)64 << 10);
+    if (host) cudaFreeHost(host);
+    host = nullptr;
+    cap = 0;
+    B200_CUDA(cudaHostAlloc(&host, bytes, cudaHostAllocDefault));
+    cap = bytes;
+    dev.alloc(bytes);
+  }
+  ~WriteStage() {
+    if (host) cudaFreeHost(host);
+    if (copied) cudaEventDestroy(copied);
+  }
+};
+
 enum Stage { ST_EXPAND = 0, ST_MUL, ST_FROMNTT, ST_FOLD, ST_PACK, ST_ENCODE, ST_QIMG /* query operand re-tiling */, ST_COUNT };
 
 }  // namespace
@@ -118,6 +150,8 @@ struct b200pir_ctx {
   size_t folded_stride = 0;           // u32 words between consecutive (query, slice) survivors
   DevBuf<uint64_t> w_packed;     // [Q][inst][n+1][n][2048]
   DevBuf<uint8_t> w_resp;        // [Q][response_bytes]
+  WriteStage wstage[2];          // staging of the write path, used alternately
+  int wnext = 0;
   // Coalescing of concurrent callers ("coalesce", default on): lib/server takes a READ lock around process_query
   // (bin/server.rs:102), so actix workers call it concurrently.  Requests arriving while a batch runs queue up here; the
   // thread that finds no batch in flight becomes the leader and serves everything queued (up to kCoalesceMax) in ONE
@@ -250,6 +284,21 @@ struct b200pir_db {
     if (nv != h_tile_mask[w]) {
       h_tile_mask[w] = nv;
       B200_CUDA(cudaMemcpyAsync(tile_mask.p + w, &h_tile_mask[w], 4, cudaMemcpyHostToDevice, s));
+    }
+  }
+  // a group of items written into every slice: host bits first, then one copy of the changed tile-mask range per slice
+  void mark_many(const ItemWrite* items, size_t count, cudaStream_t s) {
+    for (int slice = 0; slice < ctx->slices; slice++) {
+      size_t lo = SIZE_MAX, hi = 0;
+      for (size_t k = 0; k < count; k++) {
+        const uint64_t bit = ((uint64_t)slice * rows + items[k].il) * ctx->dim0 + items[k].j;
+        if (!((present[bit >> 6] >> (bit & 63)) & 1)) { present[bit >> 6] |= 1ull << (bit & 63); present_count++; }
+        const size_t w = (size_t)slice * T.mt + (items[k].il >> 5);
+        const uint32_t nv = h_tile_mask[w] | (1u << (items[k].j >> 5));
+        if (nv != h_tile_mask[w]) { h_tile_mask[w] = nv; lo = std::min(lo, w); hi = std::max(hi, w); }
+      }
+      if (lo <= hi)
+        B200_CUDA(cudaMemcpyAsync(tile_mask.p + lo, &h_tile_mask[lo], (hi - lo + 1) * 4, cudaMemcpyHostToDevice, s));
     }
   }
   // a whole slice written at once (bulk upload, file load, synthetic fill): every item of it exists from now on
@@ -868,50 +917,137 @@ int b200pir_db_upsert_item(b200pir_ctx* c, b200pir_db* db, uint64_t slice, uint6
   B200_CUDA(cudaStreamSynchronize(c->stream));
   API_END
 }
+extern "C++" {
+namespace {
+// bytes_per_chunk of the raw write paths (convert_pt_to_poly asserts logp == 8, loading.rs:291; chunks fit a polynomial)
+size_t write_chunk_bytes(b200pir_ctx* c) {
+  if (c->hp.p != 256) throw Error(B200PIR_E_UNSUPPORTED, "convert_pt_to_poly asserts logp == 8 (loading.rs:291)");
+  const size_t chunks = (size_t)c->slices;
+  const size_t bpc = (c->hp.db_item_size + chunks - 1) / chunks;            // params.bytes_per_chunk()
+  if (bpc > (size_t)POLY) throw Error(B200PIR_E_SHAPE, "bytes_per_chunk exceeds poly_len");           // server.rs:292
+  return bpc;
+}
+// One group of distinct items (their raw bytes: `data_bytes` filled by fill(dst); items[k].off relative to dst) converted and
+// placed by one launch of the fused kernel, staged through the context's next pinned / device buffer pair.  Stream-ordered:
+// the caller synchronises.
+template <typename Fill>
+void write_group(b200pir_ctx* c, b200pir_db* db, const std::vector<ItemWrite>& items, size_t data_bytes, Fill fill) {
+  if (items.empty()) return;
+  WriteStage& st = c->wstage[c->wnext];
+  c->wnext ^= 1;
+  const size_t head = (items.size() * sizeof(ItemWrite) + 15) & ~(size_t)15;
+  st.ensure(head + data_bytes);
+  std::memcpy(st.host, items.data(), items.size() * sizeof(ItemWrite));
+  fill(st.host + head);
+  B200_CUDA(cudaMemcpyAsync(st.dev.p, st.host, head + data_bytes, cudaMemcpyHostToDevice, c->stream));
+  B200_CUDA(cudaEventRecord(st.copied, c->stream));
+  const ItemWrite* d_items = reinterpret_cast<const ItemWrite*>(st.dev.p);
+  const uint8_t* d_data = st.dev.p + head;
+  const int bpc = (int)write_chunk_bytes(c), count = (int)items.size();
+  if (db->format == 0) launch_write_items(c->dp, c->geom(db->rows), db->d.p, c->slices, d_items, count, d_data, bpc, c->hp.p, c->stream);
+  else if (db->format == 2) launch_write_items(c->dp, db->T, db->t.p, c->slices, d_items, count, d_data, bpc, c->hp.p, c->stream);
+  else launch_write_items(c->dp, db->F, db->f.p, c->slices, d_items, count, d_data, bpc, c->hp.p, c->stream);
+  B200_CUDA(cudaGetLastError());
+}
+uint32_t load_be32(const uint8_t* p) { return ((uint32_t)p[0] << 24) | ((uint32_t)p[1] << 16) | ((uint32_t)p[2] << 8) | p[3]; }
+}  // namespace
+}  // extern "C++"
+
+// lib/server/src/db/loading.rs:361-377 update_many_items: the entries are checked and applied in body order; on a malformed
+// entry everything before it stays written.  Entries are gathered into groups (kWriteGroupItems / kWriteGroupBytes); within a
+// group only the last entry of an item is converted (the reference's serial loop leaves exactly that one), groups run in
+// order on one stream, so the last entry of an item wins across groups too.
+int b200pir_db_update_many_items(b200pir_ctx* c, b200pir_db* db, const uint8_t* body, size_t len, uint64_t* largest_update) {
+  API_BEGIN
+  if (!c || (!body && len)) throw Error(B200PIR_E_BADARG, "null argument");
+  Guard gd(c);
+  check_db(c, db);
+  const size_t bpc = write_chunk_bytes(c);
+  const size_t max_data = (size_t)c->slices * bpc;
+  const uint64_t num_items = (uint64_t)c->dim0 * c->num_per;
+  struct Entry { size_t off; uint32_t len, idx; };
+  std::vector<Entry> group;
+  size_t group_bytes = 0;
+  std::vector<ItemWrite> items;
+  std::vector<size_t> src;                                                  // body offset of items[k]'s bytes
+  std::unordered_set<uint32_t> seen;
+  auto flush = [&]() {
+    items.clear();
+    src.clear();
+    seen.clear();
+    size_t bytes = 0;
+    for (size_t k = group.size(); k-- > 0;) {                               // last occurrence first
+      const Entry& e = group[k];
+      if (!seen.insert(e.idx).second) continue;
+      const int ii = (int)(e.idx % c->num_per), j = (int)(e.idx / c->num_per);
+      items.push_back(ItemWrite{(uint32_t)bytes, e.len, (uint32_t)(ii / db->shard.count), (uint32_t)j});
+      src.push_back(e.off);
+      bytes += e.len;
+    }
+    write_group(c, db, items, bytes, [&](uint8_t* dst) {
+      for (size_t k = 0; k < items.size(); k++) std::memcpy(dst + items[k].off, body + src[k], items[k].len);
+    });
+    db->mark_many(items.data(), items.size(), c->stream);
+    group.clear();
+    group_bytes = 0;
+  };
+  std::string err;
+  uint64_t largest = 0;
+  size_t offs = 0;
+  while (offs < len) {
+    if (len - offs < 4) { err = "truncated entry length"; break; }
+    const uint32_t chunk_len = load_be32(body + offs);
+    if (chunk_len > len - offs - 4) { err = "entry runs past the end of the body"; break; }
+    largest = std::max<uint64_t>(largest, chunk_len);
+    if (chunk_len > 4 + max_data) { err = "update longer than instances*n^2*bytes_per_chunk"; break; }   // loading.rs:308-310
+    if (chunk_len < 4) { err = "entry shorter than its db_idx"; break; }
+    const uint32_t idx = load_be32(body + offs + 4);
+    if (idx >= num_items) { err = "bad db idx"; break; }                                               // loading.rs:333-340
+    if ((idx % c->num_per) % db->shard.count == (uint64_t)db->shard.index) {   // else the row lives on another GPU
+      group.push_back(Entry{offs + 8, chunk_len - 4, idx});
+      group_bytes += chunk_len - 4;
+      if (group.size() == kWriteGroupItems || group_bytes >= kWriteGroupBytes) flush();
+    }
+    offs += 4 + (size_t)chunk_len;
+  }
+  flush();
+  // the host RwLock gives writers exclusive access (bin/server.rs:31-43): readers see the body applied up to `err`, never less
+  B200_CUDA(cudaStreamSynchronize(c->stream));
+  if (!err.empty()) throw Error(B200PIR_E_SHAPE, err);
+  if (largest_update) *largest_update = largest;
+  API_END
+}
+
 int b200pir_db_update_item_raw(b200pir_ctx* c, b200pir_db* db, uint64_t db_idx, const uint8_t* data, size_t len) {
   API_BEGIN
   if (!c || (!data && len)) throw Error(B200PIR_E_BADARG, "null argument");
   Guard gd(c);
   check_db(c, db);
-  const auto& hp = c->hp;
-  if (hp.p != 256) throw Error(B200PIR_E_UNSUPPORTED, "convert_pt_to_poly asserts logp == 8 (loading.rs:291)");
-  const size_t chunks = (size_t)c->slices;
-  const size_t pt_len = (hp.db_item_size + chunks - 1) / chunks;            // params.bytes_per_chunk()
-  if (pt_len > (size_t)POLY) throw Error(B200PIR_E_SHAPE, "bytes_per_chunk exceeds poly_len");
-  if (len > chunks * pt_len) throw Error(B200PIR_E_SHAPE, "update longer than instances*n^2*bytes_per_chunk");   // loading.rs:308-310
+  const size_t bpc = write_chunk_bytes(c);
+  if (len > (size_t)c->slices * bpc) throw Error(B200PIR_E_SHAPE, "update longer than instances*n^2*bytes_per_chunk");   // loading.rs:308-310
   if (db_idx >= (uint64_t)c->dim0 * c->num_per) throw Error(B200PIR_E_SHAPE, "bad db idx");                      // loading.rs:333-340
   const int ii = (int)(db_idx % c->num_per), j = (int)(db_idx / c->num_per);
   if (ii % db->shard.count != db->shard.index) return 0;                      // row lives on another GPU
-  DevBuf<uint8_t> bucket(chunks * pt_len);
-  DevBuf<uint64_t> polys(chunks * POLY);
-  B200_CUDA(cudaMemsetAsync(bucket.p, 0, bucket.n, c->stream));
-  if (len) B200_CUDA(cudaMemcpyAsync(bucket.p, data, len, cudaMemcpyHostToDevice, c->stream));
-  launch_item_from_bytes(c->dp, bucket.p, (int)chunks, (int)pt_len, hp.p, polys.p, c->stream);
-  for (size_t s = 0; s < chunks; s++) {
-    if (db->format == 0) launch_db_upsert(c->geom(db->rows), db->d.p, (int)s, ii / db->shard.count, j, polys.p + s * POLY, c->stream);
-    else if (db->format == 2) launch_db_upsert_tc5(db->T, db->t.p, (int)s, ii / db->shard.count, j, polys.p + s * POLY, c->stream);
-    else launch_db_upsert_frag(db->F, db->f.p, (int)s, ii / db->shard.count, j, polys.p + s * POLY, c->stream);
-    db->mark((int)s, ii / db->shard.count, j, c->stream);
-  }
+  const std::vector<ItemWrite> items{ItemWrite{0, (uint32_t)len, (uint32_t)(ii / db->shard.count), (uint32_t)j}};
+  write_group(c, db, items, len, [&](uint8_t* dst) { if (len) std::memcpy(dst, data, len); });
+  db->mark_many(items.data(), 1, c->stream);
   B200_CUDA(cudaStreamSynchronize(c->stream));                                // writers hold the host write lock
-  B200_CUDA(cudaGetLastError());
   API_END
 }
 
 // load_db_from_seek (lib/spiral-rs/src/server.rs:277-357; lib/server/src/db/loading.rs:192-247): `path` is the raw database,
 // item i at byte i * db_item_size.  Chunk c of item i is the bytes_per_chunk bytes at i * db_item_size + c * bytes_per_chunk,
 // clipped at the end of the FILE (as the reference's read does), each byte one plaintext coefficient; items past the end
-// of the file are zero polynomials.  Conversion (recenter, NTT, pack) and placement run on the GPU, `group` items per launch.
+// of the file are zero polynomials.  So item i is the update_item_raw of the file's bytes [i * db_item_size, + chunks *
+// bytes_per_chunk), clipped at its end: one read per group of items, whose ranges may overlap, converted and placed by the
+// fused kernel.
 int b200pir_db_load_raw_file(b200pir_ctx* c, b200pir_db* db, const char* path) {
   API_BEGIN
   if (!c || !path) throw Error(B200PIR_E_BADARG, "null argument");
   Guard gd(c);
   check_db(c, db);
-  const auto& hp = c->hp;
-  if (hp.p != 256) throw Error(B200PIR_E_UNSUPPORTED, "load_item_from_seek is restated for logp == 8 only");
-  const size_t chunks = (size_t)c->slices;
-  const size_t bpc = (hp.db_item_size + chunks - 1) / chunks;                // params.bytes_per_chunk()
-  if (bpc > (size_t)POLY) throw Error(B200PIR_E_SHAPE, "bytes_per_chunk exceeds poly_len");     // server.rs:292
+  const size_t bpc = write_chunk_bytes(c);
+  const size_t span = (size_t)c->slices * bpc, isz = c->hp.db_item_size;
   struct Closer { FILE* f; ~Closer() { if (f) fclose(f); } } file{fopen(path, "rb")};
   if (!file.f) throw Error(B200PIR_E_BADARG, std::string("cannot open ") + path);
   if (fseeko(file.f, 0, SEEK_END)) throw Error(B200PIR_E_BADARG, "cannot seek in the database file");
@@ -919,34 +1055,23 @@ int b200pir_db_load_raw_file(b200pir_ctx* c, b200pir_db* db, const char* path) {
   if (fbytes < 0) throw Error(B200PIR_E_BADARG, "cannot size the database file");
   const size_t flen = (size_t)fbytes;
   const size_t num_items = (size_t)c->dim0 * c->num_per;
-  const size_t group = 64;                                                    // items converted per launch
-  std::vector<uint8_t> host(group * chunks * bpc);
-  DevBuf<uint8_t> bucket(group * chunks * bpc);
-  DevBuf<uint64_t> polys(group * chunks * POLY);
+  const size_t group = std::max<size_t>(1, std::min(kWriteGroupItems, (kWriteGroupBytes - std::min(span, kWriteGroupBytes)) / std::max<size_t>(isz, 1) + 1));
+  std::vector<ItemWrite> items;
   for (size_t i0 = 0; i0 < num_items; i0 += group) {
     const size_t cnt = std::min(group, num_items - i0);
-    std::fill(host.begin(), host.end(), 0);
-    for (size_t k = 0; k < cnt; k++)
-      for (size_t ch = 0; ch < chunks; ch++) {
-        const size_t pos = (i0 + k) * hp.db_item_size + ch * bpc;
-        const size_t want = pos < flen ? std::min(bpc, flen - pos) : 0;
-        if (want && (fseeko(file.f, (off_t)pos, SEEK_SET) || fread(host.data() + (k * chunks + ch) * bpc, 1, want, file.f) != want))
-          throw Error(B200PIR_E_SHAPE, "short read from the database file");
-      }
-    B200_CUDA(cudaMemcpyAsync(bucket.p, host.data(), cnt * chunks * bpc, cudaMemcpyHostToDevice, c->stream));
-    launch_item_from_bytes(c->dp, bucket.p, (int)(cnt * chunks), (int)bpc, hp.p, polys.p, c->stream);
+    const size_t lo = std::min(i0 * isz, flen), hi = std::min((i0 + cnt - 1) * isz + span, flen);
+    items.clear();
     for (size_t k = 0; k < cnt; k++) {
-      const size_t idx = i0 + k;
+      const size_t idx = i0 + k, pos = idx * isz;
       const int ii = (int)(idx % c->num_per), j = (int)(idx / c->num_per);
       if (ii % db->shard.count != db->shard.index) continue;                  // row lives on another GPU
-      for (size_t s = 0; s < chunks; s++) {
-        const uint64_t* poly = polys.p + (k * chunks + s) * POLY;
-        if (db->format == 0) launch_db_upsert(c->geom(db->rows), db->d.p, (int)s, ii / db->shard.count, j, poly, c->stream);
-        else if (db->format == 2) launch_db_upsert_tc5(db->T, db->t.p, (int)s, ii / db->shard.count, j, poly, c->stream);
-        else launch_db_upsert_frag(db->F, db->f.p, (int)s, ii / db->shard.count, j, poly, c->stream);
-      }
+      const size_t have = pos < flen ? std::min(span, flen - pos) : 0;
+      items.push_back(ItemWrite{(uint32_t)(have ? pos - lo : 0), (uint32_t)have, (uint32_t)(ii / db->shard.count), (uint32_t)j});
     }
-    B200_CUDA(cudaStreamSynchronize(c->stream));                              // `host` is refilled next
+    write_group(c, db, items, hi - lo, [&](uint8_t* dst) {
+      if (hi > lo && (fseeko(file.f, (off_t)lo, SEEK_SET) || fread(dst, 1, hi - lo, file.f) != hi - lo))
+        throw Error(B200PIR_E_SHAPE, "short read from the database file");
+    });
   }
   for (int s = 0; s < c->slices; s++) db->mark_slice(s, c->stream);            // load_db_from_seek builds a dense database
   B200_CUDA(cudaStreamSynchronize(c->stream));

@@ -21,6 +21,7 @@
 // One CTA = one (slice, n, z): its 8 warps share the query operand B (<= 32 KiB, shared memory) and each streams
 // the fragments of two row tiles.
 #include "kernels.h"
+#include "item_write.cuh"
 
 namespace b200pir {
 
@@ -80,21 +81,29 @@ k_db_to_frag(ImmaGeom F, const uint4* __restrict__ db0_slice, uint4* __restrict_
   }
 }
 
-// one item polynomial (2048 packed words lo|hi<<32) into the fragment-order database (byte writes)
-__global__ void k_db_upsert_frag(ImmaGeom F, uint4* dbf, int slice, int il, int j, const uint64_t* poly) {
+// where word z of item (slice, local row il, j) lives in fragment order (byte writes); w = lo | hi << 32
+struct FragStore {
+  ImmaGeom F;
+  uint4* dbf;
+  __device__ __forceinline__ void operator()(int slice, int il, int j, int z, uint64_t w) const {
+    const int mt = il >> 4, row = il & 15, ks = j >> 5, k = j & 31;
+    const int g = row & 7, rh = row >> 3, kh = k >> 4, t = (k & 15) >> 2, i = k & 3;
+    const int lane = g * 4 + t, reg = rh + 2 * kh;     // a0..a3 = (row g,k lo), (row g+8,k lo), (row g,k hi), (row g+8,k hi)
+#pragma unroll
+    for (int n = 0; n < 2; n++) {
+      uint32_t r = n ? (uint32_t)(w >> 32) : (uint32_t)w;
+      uint8_t* base = reinterpret_cast<uint8_t*>(dbf + (((((size_t)slice * 2 + n) * POLY + z) * F.mt + mt) * F.ks + ks) * 4 * 32);
+#pragma unroll
+      for (int l = 0; l < 4; l++) base[((size_t)l * 32 + lane) * 16 + reg * 4 + i] = (uint8_t)((r >> (7 * l)) & 127u);
+    }
+  }
+};
+
+// one item polynomial (2048 packed words lo|hi<<32) into the fragment-order database
+__global__ void k_db_upsert_frag(FragStore st, int slice, int il, int j, const uint64_t* poly) {
   int z = blockIdx.x * blockDim.x + threadIdx.x;
   if (z >= POLY) return;
-  const int mt = il >> 4, row = il & 15, ks = j >> 5, k = j & 31;
-  const int g = row & 7, rh = row >> 3, kh = k >> 4, t = (k & 15) >> 2, i = k & 3;
-  const int lane = g * 4 + t, reg = rh + 2 * kh;       // a0..a3 = (row g,k lo), (row g+8,k lo), (row g,k hi), (row g+8,k hi)
-  uint64_t w = poly[z];
-#pragma unroll
-  for (int n = 0; n < 2; n++) {
-    uint32_t r = n ? (uint32_t)(w >> 32) : (uint32_t)w;
-    uint8_t* base = reinterpret_cast<uint8_t*>(dbf + (((((size_t)slice * 2 + n) * POLY + z) * F.mt + mt) * F.ks + ks) * 4 * 32);
-#pragma unroll
-    for (int l = 0; l < 4; l++) base[((size_t)l * 32 + lane) * 16 + reg * 4 + i] = (uint8_t)((r >> (7 * l)) & 127u);
-  }
+  st(slice, il, j, z, poly[z]);
 }
 
 // expanded queries (format of mul_kernels.cu: uint4 [jp][jb][z]) -> B fragments
@@ -474,7 +483,11 @@ void launch_db_to_frag(const ImmaGeom& F, const uint4* db0_slice, uint4* dbf, in
 }
 void launch_db_upsert_frag(const ImmaGeom& F, uint4* dbf, int slice, int il, int j, const uint64_t* poly, cudaStream_t s) {
   ++g_kernel_launches;
-  k_db_upsert_frag<<<POLY / 256, 256, 0, s>>>(F, dbf, slice, il, j, poly);
+  k_db_upsert_frag<<<POLY / 256, 256, 0, s>>>(FragStore{F, dbf}, slice, il, j, poly);
+}
+void launch_write_items(const DevParams& P, const ImmaGeom& F, uint4* dbf, int slices, const ItemWrite* items, int count,
+                        const uint8_t* data, int bpc, uint64_t pt_modulus, cudaStream_t s) {
+  item_write::launch(P, FragStore{F, dbf}, items, count, slices, data, bpc, pt_modulus, s);
 }
 void launch_query_to_frag(const ImmaGeom& F, const uint4* q_dev, size_t q_stride, int nq, uint2* qf, cudaStream_t s) {
   const int ntiles = imma_query_tiles(nq);

@@ -72,9 +72,13 @@ void launch_db_retile_chunk(const MulGeom& G, Shard sh, uint4* db_dev_slice, con
                             cudaStream_t s);
 // one item poly (2048 packed words, lo|hi<<32) -> its place in db_dev   (lib/server db/loading.rs:317-359)
 void launch_db_upsert(const MulGeom& G, uint4* db_dev, int slice, int il, int j, const uint64_t* poly, cudaStream_t s);
-// lib/server db/loading.rs:278-299,34-41: `chunks` chunks of pt_len bytes -> packed item polynomials [chunks][2048]
-void launch_item_from_bytes(const DevParams& P, const uint8_t* bucket, int chunks, int pt_len, uint64_t pt_modulus,
-                            uint64_t* out, cudaStream_t s);
+// One item of a bulk write (item_write.cuh): its raw bytes are data[off, off + len), zero padded to slices * bpc; it goes to
+// local row il, column j of every slice.
+struct ItemWrite { uint32_t off, len, il, j; };
+// lib/server db/loading.rs:317-359 update_item_raw for `count` distinct items in one launch (raw bytes -> recenter, NTT, pack
+// -> the database layout); one overload per layout
+void launch_write_items(const DevParams& P, const MulGeom& G, uint4* db_dev, int slices, const ItemWrite* items, int count,
+                        const uint8_t* data, int bpc, uint64_t pt_modulus, cudaStream_t s);
 // synthetic DB: plaintext coeff = splitmix64(seed, ((slice*items + item)*2048 + z)) % p, recentred, NTT'd, packed
 // (server.rs:223-275 with a counter PRNG; item = j*num_per_global + ii)
 void launch_db_synth(const DevParams& P, const MulGeom& G, Shard sh, uint4* db_dev, uint64_t seed, uint64_t pt_modulus,
@@ -91,6 +95,8 @@ void upload_imma_constants(const Twiddle* lo);
 // one slice in the IMAD layout (uint4 [row][jp][z]) -> fragment order
 void launch_db_to_frag(const ImmaGeom& F, const uint4* db0_slice, uint4* dbf, int slice, cudaStream_t s);
 void launch_db_upsert_frag(const ImmaGeom& F, uint4* dbf, int slice, int il, int j, const uint64_t* poly, cudaStream_t s);
+void launch_write_items(const DevParams& P, const ImmaGeom& F, uint4* dbf, int slices, const ItemWrite* items, int count,
+                        const uint8_t* data, int bpc, uint64_t pt_modulus, cudaStream_t s);
 void launch_query_to_frag(const ImmaGeom& F, const uint4* q_dev, size_t q_stride, int nq, uint2* qf, cudaStream_t s);
 // out_zm: u32 [query][slice][n][z][row][ct_row]  (queries out_stride words apart)
 void launch_multiply_imma(const DevParams& P, const ImmaGeom& F, const uint4* dbf, const uint2* qf, uint32_t* out_zm,
@@ -108,6 +114,8 @@ size_t tc5_query_bytes(const Tc5Geom& T);                 // 16 queries
 bool tc5_supported(const Tc5Geom& T);
 void launch_db_to_tc5(const Tc5Geom& T, const uint4* db0_slice, uint8_t* dbt, int slice, cudaStream_t s);
 void launch_db_upsert_tc5(const Tc5Geom& T, uint8_t* dbt, int slice, int il, int j, const uint64_t* poly, cudaStream_t s);
+void launch_write_items(const DevParams& P, const Tc5Geom& T, uint8_t* dbt, int slices, const ItemWrite* items, int count,
+                        const uint8_t* data, int bpc, uint64_t pt_modulus, cudaStream_t s);
 void launch_query_to_tc5(const Tc5Geom& T, const uint4* q_dev, size_t q_stride, int nq, uint8_t* qt, cudaStream_t s);
 // out_zm as launch_multiply_imma; up to 16 queries per pass; one persistent CTA per SM
 // reorient_reg_ciphertexts (util.rs:323-355) fused with the re-tiling: expansion workspace v (ntt32 [query][slot][row][n][z]) ->

@@ -13,6 +13,7 @@
 // in registers.  Products are < 2^56, so the sums are reduced mod q_n every 256 terms (the reference
 // accumulates in u128 and reduces once; both give the canonical residue).
 #include "kernels.h"
+#include "item_write.cuh"
 #include <algorithm>
 
 namespace b200pir {
@@ -154,13 +155,21 @@ __global__ void k_db_retile(MulGeom G, Shard sh, uint4* db_slice, const uint64_t
       make_uint4((uint32_t)w0, (uint32_t)(w0 >> 32), (uint32_t)w1, (uint32_t)(w1 >> 32));
 }
 
-__global__ void k_db_upsert(MulGeom G, uint4* db, int slice, int ii, int j, const uint64_t* poly) {
+// where word z of item (slice, local row il, j) lives in the IMAD layout; w = lo | hi << 32
+struct ImadStore {
+  MulGeom G;
+  uint4* db;
+  __device__ __forceinline__ void operator()(int slice, int il, int j, int z, uint64_t w) const {
+    const int half = G.dim0 >> 1;
+    uint2* cell = reinterpret_cast<uint2*>(db + (((size_t)slice * G.num_per + il) * half + (j >> 1)) * POLY + z) + (j & 1);
+    *cell = make_uint2((uint32_t)w, (uint32_t)(w >> 32));
+  }
+};
+
+__global__ void k_db_upsert(ImadStore st, int slice, int il, int j, const uint64_t* poly) {
   int z = blockIdx.x * blockDim.x + threadIdx.x;
   if (z >= POLY) return;
-  const int half = G.dim0 >> 1;
-  uint2* cell = reinterpret_cast<uint2*>(db + (((size_t)slice * G.num_per + ii) * half + (j >> 1)) * POLY + z) + (j & 1);
-  uint64_t w = poly[z];
-  *cell = make_uint2((uint32_t)w, (uint32_t)(w >> 32));
+  st(slice, il, j, z, poly[z]);
 }
 
 __device__ __forceinline__ uint64_t splitmix64_at(uint64_t seed, uint64_t index) {
@@ -204,31 +213,6 @@ k_db_synth(DevParams P, MulGeom G, Shard sh, uint4* db, uint64_t seed, uint64_t 
   uint4* dst = db + (((size_t)slice * G.num_per + ii) * half + jp) * POLY;
   const uint4* c4 = reinterpret_cast<const uint4*>(cell);
   for (int z = threadIdx.x; z < POLY; z += 512) dst[z] = c4[z];
-}
-
-// lib/server/src/db/loading.rs:278-299 convert_pt_to_poly + :34-41 pack_ntt_poly for every chunk of one bucket:
-// chunk c (pt_len bytes of `bucket`, zero padded) -> out[c][z] = ntt(coeffs).lo | .hi << 32.  grid = chunks, 512 threads.
-__global__ void __launch_bounds__(512, 1)
-k_item_from_bytes(DevParams P, const uint8_t* __restrict__ bucket, int pt_len, uint64_t pt, uint64_t* __restrict__ out) {
-  __shared__ __align__(16) uint32_t ntt_smem[2 * NTT_SMEM_WORDS];
-  __shared__ uint32_t halves[2][POLY];
-  const int n = threadIdx.x >> 8, tid = threadIdx.x & 255;
-  const uint32_t q = n ? P.q[1] : P.q[0];
-  const uint8_t* src = bucket + (size_t)blockIdx.x * pt_len;
-  struct S { __device__ __forceinline__ void operator()() const { __syncthreads(); } };
-  uint32_t x[8];
-#pragma unroll
-  for (int a = 0; a < 8; a++) {
-    const int i = a * 256 + tid;
-    const uint64_t v = i < pt_len ? (uint64_t)src[i] : 0;
-    x[a] = (v > pt / 2) ? (uint32_t)(q - (uint32_t)(pt - v)) : (uint32_t)v;       // recenter_mod, then mod q_n
-  }
-  ntt_forward_group_lz<NTT_OUT_CANON>(tid, x, ntt_smem + n * NTT_SMEM_WORDS, TwConstM{n, 0}, TwGlobalM{n ? P.fwd[1] : P.fwd[0]}, q, S());   // inputs canonical
-#pragma unroll
-  for (int k = 0; k < 8; k++) halves[n][tid * 8 + k] = x[k];
-  __syncthreads();
-  for (int z = threadIdx.x; z < POLY; z += 512)
-    out[(size_t)blockIdx.x * POLY + z] = (uint64_t)halves[0][z] | ((uint64_t)halves[1][z] << 32);
 }
 
 // ------------------------------------------------------------------ DoublePIR
@@ -454,12 +438,11 @@ void launch_db_retile_chunk(const MulGeom& G, Shard sh, uint4* db_dev_slice, con
 }
 void launch_db_upsert(const MulGeom& G, uint4* db_dev, int slice, int il, int j, const uint64_t* poly, cudaStream_t s) {
   ++g_kernel_launches;
-  k_db_upsert<<<POLY / 256, 256, 0, s>>>(G, db_dev, slice, il, j, poly);
+  k_db_upsert<<<POLY / 256, 256, 0, s>>>(ImadStore{G, db_dev}, slice, il, j, poly);
 }
-void launch_item_from_bytes(const DevParams& P, const uint8_t* bucket, int chunks, int pt_len, uint64_t pt_modulus,
-                            uint64_t* out, cudaStream_t s) {
-  ++g_kernel_launches;
-  k_item_from_bytes<<<chunks, 512, 0, s>>>(P, bucket, pt_len, pt_modulus, out);
+void launch_write_items(const DevParams& P, const MulGeom& G, uint4* db_dev, int slices, const ItemWrite* items, int count,
+                        const uint8_t* data, int bpc, uint64_t pt_modulus, cudaStream_t s) {
+  item_write::launch(P, ImadStore{G, db_dev}, items, count, slices, data, bpc, pt_modulus, s);
 }
 void launch_db_synth(const DevParams& P, const MulGeom& G, Shard sh, uint4* db_dev, uint64_t seed, uint64_t pt_modulus,
                      int slice_begin, int slice_count, cudaStream_t s) {

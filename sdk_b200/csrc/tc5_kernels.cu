@@ -29,6 +29,7 @@
 // of the TMEM loads, shuffles and wide multiplies).  Pipelines: A ring (full/empty mbarriers), double-buffered B operand
 // (bfull/bempty), double-buffered accumulator in TMEM (tfull/tempty).
 #include "kernels.h"
+#include "item_write.cuh"
 #include "tc5_ptx.cuh"
 #include <cstdio>
 #include <cstdlib>
@@ -64,19 +65,27 @@ k_db_to_tc5(Tc5Geom T, const uint4* __restrict__ db0_slice, uint8_t* __restrict_
   for (int n = 0; n < 2; n++) tc5_db_store(dbt + tc5_db_tile(T, slice, n, z, mt, ks) * TC5_TILE, t, res[n]);
 }
 
-// one item polynomial (2048 packed words lo|hi<<32) into the tile images (byte writes)
-__global__ void k_db_upsert_tc5(Tc5Geom T, uint8_t* dbt, int slice, int il, int j, const uint64_t* poly) {
+// where word z of item (slice, local row il, j) lives in the tile images (byte writes); w = lo | hi << 32
+struct Tc5Store {
+  Tc5Geom T;
+  uint8_t* dbt;
+  __device__ __forceinline__ void operator()(int slice, int il, int j, int z, uint64_t w) const {
+    const int mt = il >> 5, row_local = il & 31, ks = j >> 5, k = j & 31;
+#pragma unroll
+    for (int n = 0; n < 2; n++) {
+      const uint32_t r = n ? (uint32_t)(w >> 32) : (uint32_t)w;
+      uint8_t* tile = dbt + tc5_db_tile(T, slice, n, z, mt, ks) * TC5_TILE;
+#pragma unroll
+      for (int l = 0; l < 4; l++) tile[tc5_tile_off(tc5_m_index(row_local, l), k)] = (uint8_t)((r >> (7 * l)) & 127u);
+    }
+  }
+};
+
+// one item polynomial (2048 packed words lo|hi<<32) into the tile images
+__global__ void k_db_upsert_tc5(Tc5Store st, int slice, int il, int j, const uint64_t* poly) {
   const int z = blockIdx.x * blockDim.x + threadIdx.x;
   if (z >= POLY) return;
-  const int mt = il >> 5, row_local = il & 31, ks = j >> 5, k = j & 31;
-  const uint64_t w = poly[z];
-#pragma unroll
-  for (int n = 0; n < 2; n++) {
-    const uint32_t r = n ? (uint32_t)(w >> 32) : (uint32_t)w;
-    uint8_t* tile = dbt + tc5_db_tile(T, slice, n, z, mt, ks) * TC5_TILE;
-#pragma unroll
-    for (int l = 0; l < 4; l++) tile[tc5_tile_off(tc5_m_index(row_local, l), k)] = (uint8_t)((r >> (7 * l)) & 127u);
-  }
+  st(slice, il, j, z, poly[z]);
 }
 
 // expanded queries (uint4 [j][z] per query, q_stride apart) -> qT.  CTA = (pair of z, ks): every 32-byte sector it reads is
@@ -377,7 +386,11 @@ void launch_db_to_tc5(const Tc5Geom& T, const uint4* db0_slice, uint8_t* dbt, in
 }
 void launch_db_upsert_tc5(const Tc5Geom& T, uint8_t* dbt, int slice, int il, int j, const uint64_t* poly, cudaStream_t s) {
   ++g_kernel_launches;
-  k_db_upsert_tc5<<<POLY / 256, 256, 0, s>>>(T, dbt, slice, il, j, poly);
+  k_db_upsert_tc5<<<POLY / 256, 256, 0, s>>>(Tc5Store{T, dbt}, slice, il, j, poly);
+}
+void launch_write_items(const DevParams& P, const Tc5Geom& T, uint8_t* dbt, int slices, const ItemWrite* items, int count,
+                        const uint8_t* data, int bpc, uint64_t pt_modulus, cudaStream_t s) {
+  item_write::launch(P, Tc5Store{T, dbt}, items, count, slices, data, bpc, pt_modulus, s);
 }
 void launch_query_to_tc5(const Tc5Geom& T, const uint4* q_dev, size_t q_stride, int nq, uint8_t* qt, cudaStream_t s) {
   if (nq < 1 || nq > 16) throw Error(-2, "tcgen05 multiply: 1..16 queries per pass");

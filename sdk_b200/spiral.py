@@ -162,6 +162,16 @@ class Database:
         data = np.ascontiguousarray(data, dtype=np.uint8)
         check(LIB.b200pir_db_update_item_raw(self.params._h, self._h, db_idx, data.ctypes.data, data.size))
 
+    def update_many_items(self, body):
+        """lib/server/src/db/loading.rs:361-377 (the /update-row body): entries [u32 BE chunk_len][u32 BE db_idx][data]
+        applied in order, the last entry of an item winning; returns largest_update (the longest chunk_len).  body: bytes or
+        a uint8 array.  A malformed entry raises B200PirError with the entries before it written."""
+        body = np.frombuffer(body, dtype=np.uint8) if isinstance(body, (bytes, bytearray, memoryview)) else \
+            np.ascontiguousarray(body, dtype=np.uint8)
+        largest = C.c_uint64(0)
+        check(LIB.b200pir_db_update_many_items(self.params._h, self._h, body.ctypes.data, body.size, C.byref(largest)))
+        return largest.value
+
     def fill_synthetic(self, seed):
         check(LIB.b200pir_db_fill_synthetic(self.params._h, self._h, seed))
 
